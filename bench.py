@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the B200-native scan->pointcloud path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--only k1|k2|sweep]
+                    [--dump-outputs DIR]
 
 ONE JSON line (the last line of stdout).  Top level = BASELINE.json's metric on configs[1]:
 Mpoints/s of 128x2048 dual-return range->XYZ (+ destaggered range) through the fused K1 kernel, with
@@ -15,7 +16,12 @@ Mpoints/s of 128x2048 dual-return range->XYZ (+ destaggered range) through the f
 
 A "step" is one pass of the hot path over one batch of `frames_per_step` synthetic frames (K1: 128 frames
 = 67 Mpoints and 1.35 GB of DRAM traffic per step; K2: 32 frames, 0.57 GB -- far beyond the 126 MB L2, so
-consecutive steps cannot be served from cache).
+consecutive steps cannot be served from cache).  --steps sets the number of timed steps of every record.
+
+--dump-outputs DIR writes what the last timed K1 and K2 steps computed (rank 0) as DIR/<name>.npy: XYZ and
+destaggered range of K1; the fields, XYZ, destaggered ranges and column headers of K2.  Each is a fixed,
+seeded sample of the output (float32, or float64 where float32 would round), and the inputs are seeded, so
+two builds run with the same arguments can be compared array for array.
 
   value : device-resident inputs/outputs, one fused launch per step, CUDA-event timed.
   e2e   : the same batch through the C ABI with HOST (pinned) buffers: H2D of the inputs and D2H of
@@ -52,6 +58,7 @@ POINTS_PER_FRAME = H * W * R
 SHIFTS = np.tile(np.array([48, 32, 16, 0], np.int32), H // 4)  # OS1-128 1024-mode shifts x2 (SURVEY 8d)
 K1_WORKLOAD = "OS1-128 2048x128 dual-return fused destagger+cartesian (K1), LUT tiles staged in smem via TMA"
 METRIC = "Mpoints/s 128x2048 dual-return range->XYZ"
+DUMP_K1_POINTS = 1 << 20               # --dump-outputs: 20 MB of K1 points (XYZ + destaggered range)
 
 # kept for tools/ that import them
 K1_BYTES_PER_FRAME_F32 = 16_777_216     # SURVEY 8(d) algorithmic: 64 B/px = 8 (range) + 24 (LUT) + 24 (xyz) + 8 (rd)
@@ -171,8 +178,9 @@ def bind_to_gpu_numa(local_rank):
     return 0
 
 
-def measure_k1(args, ob, torch, dist, rank, local_rank, world, pcie):
-    """configs[1]: the top-level record."""
+def measure_k1(args, ob, torch, dist, rank, local_rank, world, pcie, dump=None):
+    """configs[1]: the top-level record.  With a `dump` dict, rank 0 adds to it a seeded sample of the
+    points its last timed step computed."""
     dev = torch.device("cuda", local_rank)
     F = args.frames
     # ---- inputs: each rank owns F independent frames (one "sensor stream shard") ----
@@ -213,6 +221,10 @@ def measure_k1(args, ob, torch, dist, rank, local_rank, world, pcie):
     sampler.mark()
     launches = ob.kernel_launch_count() - l0
     clocks = sampler.stop()
+    if dump is not None and rank == 0:
+        idx = bc.dump_index(torch, dev, F * R * H * W, DUMP_K1_POINTS, seed=1)
+        dump["k1_xyz"] = bc.dump_array(t_xyz.view(-1, 3)[idx], np.float32)
+        dump["k1_range_destaggered"] = bc.dump_array(t_rd.view(-1)[idx], np.uint32)
     ms_total = ev[0].elapsed_time(ev[-1])
     per_launch_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     ms_total_max = bc.max_over_ranks(torch, dist, dev, ms_total)
@@ -251,7 +263,7 @@ def measure_k1(args, ob, torch, dist, rank, local_rank, world, pcie):
             ob.scan_to_cloud(lut, SHIFTS, h_rng[sl], xyz=h_xyz[sl], range_destaggered=h_rd[sl],
                              stream=ostreams[c % NS])
 
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     for _ in range(2):
         e2e_step()
     barrier()
@@ -347,7 +359,7 @@ def measure_lut_free(args, ob, torch, dist, rank, local_rank, world):
     peak, _ = bc.measured_peaks()
     out = {}
 
-    def timed(step, steps=10, warmup=3):
+    def timed(step, warmup=3):
         bc.gpu_spin(torch, dev)
         for _ in range(warmup):
             step()
@@ -356,11 +368,11 @@ def measure_lut_free(args, ob, torch, dist, rank, local_rank, world):
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        for _ in range(steps):
+        for _ in range(args.steps):
             step()
         e1.record(stream)
         torch.cuda.synchronize()
-        return bc.max_over_ranks(torch, dist, dev, e0.elapsed_time(e1) / steps * 1e-3)
+        return bc.max_over_ranks(torch, dist, dev, e0.elapsed_time(e1) / args.steps * 1e-3)
 
     def normwise_ok(got, ref):
         err = np.linalg.norm(got.astype(np.float64) - ref.astype(np.float64), axis=-1)
@@ -430,7 +442,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--kernel-only", action="store_true", help="tuning aid: device-resident timing only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed seeded sample of what the last K1 and K2 steps "
+                         "computed to DIR/<name>.npy (float32 / float64, under 64 MB; rank 0 only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.workload:
         args.only = args.workload
@@ -461,14 +480,16 @@ def main():
         dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
 
     line = None
+    dump = {} if args.dump_outputs else None
     if args.kernel_only:
         import bench_k2
         out = {}
         if args.only in ("all", "k1"):
-            out["k1"] = measure_k1(args, ob, torch, dist, rank, local_rank, world, None)
+            out["k1"] = measure_k1(args, ob, torch, dist, rank, local_rank, world, None, dump)
         if args.only in ("all", "k2"):
             st = bench_k2.K2State(args, ob, torch, dist, rank, local_rank, world)
-            rec = bench_k2.measure_k2(st, args, args.streams_per_gpu, None, with_e2e=False, with_cpu=False)
+            rec = bench_k2.measure_k2(st, args, args.streams_per_gpu, None, with_e2e=False, with_cpu=False,
+                                      dump=dump)
             out["k2"] = {"value": rec["value"], "ms_per_step": rec["ms_per_step"], "frac": rec["roofline"]["frac"],
                          "frac_algorithmic": rec["roofline"]["frac_algorithmic"], "parity": rec["parity_vs_oracle"]["ok"],
                          "pipe_launches": rec["pipelined_kernel_launches"], "clocks": rec["clocks"]}
@@ -483,14 +504,14 @@ def main():
                     "note": "pinned 256 MB copies; with N ranks all ranks copy at the same time, so the figures "
                             "include the contention for each socket's host memory / PCIe root"}
         if args.only in ("all", "k1"):
-            line = measure_k1(args, ob, torch, dist, rank, local_rank, world, pcie)
+            line = measure_k1(args, ob, torch, dist, rank, local_rank, world, pcie, dump)
         else:
             line = {"metric": METRIC, "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "partial": args.only}
         line["pcie"] = pcie_all
         if args.only in ("all", "k2"):
             import bench_k2
             st = bench_k2.K2State(args, ob, torch, dist, rank, local_rank, world)
-            line["k2"] = bench_k2.measure_k2(st, args, 1, pcie)
+            line["k2"] = bench_k2.measure_k2(st, args, 1, pcie, dump=dump)
             line["k2_streams8"] = bench_k2.measure_k2(st, args, 8, pcie, with_e2e=False, with_cpu=False)
             del st
         if args.only == "all":
@@ -511,6 +532,8 @@ def main():
             os._exit(0)
         time.sleep(1.0)
     if rank == 0:
+        if dump is not None:
+            bc.write_dumps(args.dump_outputs, dump)
         sys.stdout.flush()
         print(json.dumps(line), flush=True)
         if dist is not None:

@@ -294,3 +294,34 @@ def all_ok(torch, dist, dev, ok):
     t = torch.tensor([1 if ok else 0], dtype=torch.int32, device=dev)
     dist.all_reduce(t, op=dist.ReduceOp.MIN)
     return bool(t.item())
+
+
+# ---------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed launches computed, as .npy files, so that two builds can be compared
+# ---------------------------------------------------------------------------------------------
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_index(torch, dev, n, k, seed):
+    """Sorted flat indices (a device tensor) of a fixed, seeded sample of k of n elements; all n when k >= n."""
+    idx = np.arange(n) if k >= n else np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+    return torch.from_numpy(idx).to(dev)
+
+
+def dump_array(t, dtype):
+    """Host copy of a device output holding `dtype` values (the tensors carry unsigned fields in signed
+    types of the same width), as float32 for floats and integers of up to 16 bits, float64 otherwise:
+    exact for every integer below 2**53."""
+    a = t.cpu().numpy().view(dtype)
+    if a.dtype.kind == "f" or a.dtype.itemsize <= 2:
+        return a.astype(np.float32)
+    return a.astype(np.float64)
+
+
+def write_dumps(directory, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)

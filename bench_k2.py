@@ -20,6 +20,8 @@ POINTS_PER_FRAME = H * W * R
 SHIFTS = np.tile(np.array([48, 32, 16, 0], np.int32), H // 4)
 PROFILE = "RNG19_RFL8_SIG16_NIR16_DUAL"
 K2_BYTES_PER_FRAME_F32 = 23_917_696   # SURVEY 8(d) algorithmic bytes (tools/)
+DUMP_K2_PIXELS = 1 << 18              # --dump-outputs: ~24 MB of K2 pixels (10 fields, XYZ and destaggered range x2)
+DUMP_K2_COLUMNS = 1 << 16             # and 1.3 MB of column headers
 
 
 def synth_packets(ob, n_distinct, seed=0xdeadbeef, profile=PROFILE, h=H, w=W, shifts=None):
@@ -116,8 +118,9 @@ class K2State:
         self.torch.cuda.synchronize()
 
 
-def measure_k2(st, args, streams_per_gpu, pcie, with_e2e=True, with_cpu=True):
-    """One K2 record (dict).  Every rank calls this; the record is complete on rank 0."""
+def measure_k2(st, args, streams_per_gpu, pcie, with_e2e=True, with_cpu=True, dump=None):
+    """One K2 record (dict).  Every rank calls this; the record is complete on rank 0.  With a `dump` dict,
+    rank 0 adds to it a seeded sample of the pixels and columns its last timed step decoded."""
     ob, torch, dist, dev = st.ob, st.torch, st.dist, st.dev
     F, world, rank = st.F, st.world, st.rank
     S = max(1, min(int(streams_per_gpu), F))
@@ -148,6 +151,18 @@ def measure_k2(st, args, streams_per_gpu, pcie, with_e2e=True, with_cpu=True):
     launches = ob.kernel_launch_count() - l0
     pipe_launches = ob.kernel_launch_count("decode_pipe") - lp0
     clocks = sampler.stop()
+    if dump is not None and rank == 0:
+        px = bc.dump_index(torch, dev, F * H * W, DUMP_K2_PIXELS, seed=2)
+        for f in st.dec.fields:
+            dump["k2_" + f["name"]] = bc.dump_array(st.fields[f["name"]].view(-1)[px],
+                                                    st.src_frames[0].field(f["name"]).dtype)
+        for r in range(R):
+            dump[f"k2_xyz{r}"] = bc.dump_array(st.xyz[r].view(-1, 3)[px], np.float32)
+            dump[f"k2_range_destaggered{r}"] = bc.dump_array(st.rd[r].view(-1)[px], np.uint32)
+        col = bc.dump_index(torch, dev, F * W, DUMP_K2_COLUMNS, seed=3)
+        dump["k2_timestamp"] = bc.dump_array(st.t_ts.view(-1)[col], np.uint64)
+        dump["k2_measurement_id"] = bc.dump_array(st.t_mid.view(-1)[col], np.uint16)
+        dump["k2_status"] = bc.dump_array(st.t_st.view(-1)[col], np.uint32)
     ms_total = ev[0].elapsed_time(ev[-1])
     per_launch_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     ms_max = bc.max_over_ranks(torch, dist, dev, ms_total)

@@ -43,7 +43,7 @@ def run_sweep(args, ob, torch, dist, rank, local_rank, world):
     orc = None
     if with_cpu:
         from oracle import oracle as orc   # CPU baseline leg only
-    steps, warmup = 20, 5
+    steps, warmup = args.steps, 5
     tdt = {1: torch.uint8, 2: torch.int16, 4: torch.int32}
     out = []
     for (h, w) in SHAPES:

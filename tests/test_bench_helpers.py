@@ -1,7 +1,11 @@
 """CPU checks of the bench plumbing (bench_common): byte accounting of the roofline objects, the traffic
-record's source hash, and the clock sampler's behaviour on a machine without NVML / nvidia-smi."""
+record's source hash, the clock sampler's behaviour on a machine without NVML / nvidia-smi, and the
+--dump-outputs helpers."""
 import json
 import os
+
+import numpy as np
+import pytest
 
 import bench_common as bc
 
@@ -54,3 +58,21 @@ def test_clock_sampler_without_gpu_reports_unavailable_or_samples():
     assert "sm_mhz" in out and "reasons" in out
     if out["sm_mhz"] is None:
         assert out.get("samples", 0) == 0 or out["reasons"] == ["unavailable"] or out.get("source") in ("nvml", "nvidia-smi")
+
+
+def test_dump_helpers_sample_reproducibly_and_convert_exactly(tmp_path):
+    """--dump-outputs: the sample is fixed by its seed, and values the device tensors carry in signed types
+    come out as the unsigned values they are, in a float type that holds them exactly."""
+    torch = pytest.importorskip("torch")
+    a, b = bc.dump_index(torch, "cpu", 1000, 100, seed=1), bc.dump_index(torch, "cpu", 1000, 100, seed=1)
+    assert torch.equal(a, b) and len(torch.unique(a)) == 100 and bool((a[1:] > a[:-1]).all())
+    assert torch.equal(bc.dump_index(torch, "cpu", 10, 100, seed=1), torch.arange(10))
+    u16 = bc.dump_array(torch.tensor([-1, 7], dtype=torch.int16), np.uint16)
+    u32 = bc.dump_array(torch.tensor([-1, 7], dtype=torch.int32), np.uint32)
+    assert u16.dtype == np.float32 and u16.tolist() == [65535.0, 7.0]
+    assert u32.dtype == np.float64 and u32.tolist() == [4294967295.0, 7.0]
+    assert bc.dump_array(torch.tensor([0.1], dtype=torch.float32), np.float32).dtype == np.float32
+    bc.write_dumps(str(tmp_path / "d"), {"x": u32})
+    assert np.array_equal(np.load(tmp_path / "d" / "x.npy"), u32)
+    with pytest.raises(SystemExit):
+        bc.write_dumps(str(tmp_path / "e"), {"big": np.zeros(bc.DUMP_MAX_BYTES // 8 + 1)})
